@@ -53,6 +53,9 @@ def parse(argv=None):
     ap.add_argument("--balance", default=os.environ.get("T4_BENCH_BALANCE", "cost"), choices=["reads", "cost"],
                     help="contiguous shards of equal read count, or of equal predicted cost (abundance model, synth.read_cost)")
     ap.add_argument("--dump-streams", default="", help="write per-stream cycles + features (npz) for cost-model calibration")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy: per read the "
+                         "return code, strand and rescue code; per contig of a fixed seeded sample the consensus, posWeight and header")
     ap.add_argument("--config", type=int, default=1, choices=[1, 3, 4],
                     help="BASELINE.json configs[] index: 1 = bulk 150 bp PE (the metric's config), 3 = 10x-style barcoded single-end "
                          "reads (whole barcodes per stream), 4 = --repseq bulk TCR-seq 100 bp SE amplicons")
@@ -71,7 +74,10 @@ def parse(argv=None):
     ap.add_argument("--assign-pass", type=int, default=int(os.environ.get("T4_BENCH_ASSIGN", 1)),
                     help="config 1: also time the AssignRead pass over the finished sets (SURVEY.md 8f-2, main.cpp:2047-2118) -- a "
                          "separate figure (`assign_pass`), outside `value` and `e2e`; 0 = skip")
-    return ap.parse_args(argv)
+    args = ap.parse_args(argv)
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs writes what a timed step computed: it needs --steps >= 1")
+    return args
 
 
 def setup_of(args):
@@ -237,6 +243,47 @@ def reference_sample(args, w, off, descs, budget_s, cores, keep=64):
             "sample": "%d of %d read shards (%d reads), uniformly sampled over the shard index range (fixed permutation), %.1f s wall "
                       "on %d threads; oracle/_ref/libt4ref.so = reference SeqSet::AddRead/RepeatAddRead/InputNovelRead driven by the "
                       "restated main.cpp loop" % (state["shards"], n_shards, state["reads"], el, cores)}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, ret, strands, resc, packed, seed=0):
+    """The results a caller of the timed step receives, as float arrays: t4_workload_results per read (return code, strand,
+    rescue code; every read while they fit half of DUMP_BYTES, else a fixed seeded sample of reads, indices in read_index)
+    and the packed contigs of every stream (t4_streams_pack_contigs), all of them or a fixed seeded sample within the rest of
+    the budget.  Contig arrays: contig_header[c] = (index in pack order, set, slot, barcode, num_read, length),
+    contig_consensus = the ASCII codes of the concatenated consensus strings, contig_pos_weight[sum(length), 4]."""
+    os.makedirs(d, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    n = len(ret)
+    idx = np.arange(n)
+    if n * 20 > DUMP_BYTES // 2:
+        idx = np.sort(rng.choice(n, size=DUMP_BYTES // 2 // 28, replace=False))
+        np.save(os.path.join(d, "read_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, "read_ret.npy"), ret[idx].astype(np.float64))
+    np.save(os.path.join(d, "read_strand.npy"), strands[idx].astype(np.float32))
+    np.save(os.path.join(d, "read_rescue.npy"), resc[idx].astype(np.float64))
+    starts = []
+    o = 0
+    while o < len(packed):
+        starts.append(o)
+        o += int(packed[o + 24:o + 28].view(np.uint32)[0])
+    budget = DUMP_BYTES - idx.nbytes * 3
+    pick = np.arange(len(starts))
+    if len(packed) * 3 > budget:        # one consensus byte -> 4 + 16 bytes of float32 output
+        pick = np.sort(rng.choice(len(starts), size=max(1, int(len(starts) * budget / (3 * len(packed)))), replace=False))
+    from trust4_b200 import dist as tdist
+    hdr, cons, pw = [], [], []
+    for c in pick:
+        o = starts[c]
+        rec = tdist.unpack_contigs(packed[o:o + int(packed[o + 24:o + 28].view(np.uint32)[0])])[0]
+        hdr.append((c, rec["set"], rec["slot"], rec["barcode"], rec["num_read"], len(rec["consensus"])))
+        cons.append(np.frombuffer(rec["consensus"].encode(), dtype=np.uint8))
+        pw.append(rec["pos_weight"])
+    np.save(os.path.join(d, "contig_header.npy"), np.array(hdr, dtype=np.float64).reshape(-1, 6))
+    np.save(os.path.join(d, "contig_consensus.npy"), np.concatenate(cons or [np.zeros(0, np.uint8)]).astype(np.float32))
+    np.save(os.path.join(d, "contig_pos_weight.npy"), np.concatenate(pw or [np.zeros((0, 4), np.int32)]).astype(np.float32))
 
 
 def build_line(args, config, value, ms_per_step, clocks, e2e, launches, roofline, roofline_probe, cpu, extra, metric="reads/sec assembled (150bp PE)"):
@@ -412,6 +459,8 @@ def main():
     clocks = sampler.stop() if sampler else None
     lib.check(lib.workload_results(wl, ret.data_ptr(), strands.data_ptr(), resc.data_ptr()))
     assembled = int((ret >= 0).sum().item() + (resc >= 0).sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ret.numpy(), strands.numpy(), resc.numpy(), pack["buf"][: merged["pack_bytes"]].cpu().numpy())
 
     # kernel-only duration of the stream kernel (one launch per step) for the roofline
     lib.check(lib.reset())

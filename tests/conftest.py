@@ -1,5 +1,4 @@
 import os
-import subprocess
 import sys
 
 import pytest
@@ -34,15 +33,9 @@ def pytest_collection_modifyitems(config, items):
 def emu_lib():
     """TEST-ONLY single-thread emulation of the device code (g++ -DT4_EMU): lets the bit-exact logic of the
     engine be checked against the oracle without a GPU.  Exports t4emu_* symbols; never shipped."""
+    import __graft_entry__
     from trust4_b200 import api
-    src = [os.path.join(ROOT, "trust4_b200", "csrc", f) for f in ("t4_api.cu", "t4_engine.h", "t4_common.h", "t4_shard.h", "t4_probe.cuh", "t4_assign.h", "t4_refscan.h", "t4_kcount.h", "t4_annot.h", "t4_readsort.h")]
-    src.append(os.path.join(ROOT, "include", "trust4_b200.h"))
-    out = os.path.join(ROOT, "tests", "emu", "libt4emu.so")
-    os.makedirs(os.path.dirname(out), exist_ok=True)
-    if not os.path.exists(out) or any(os.path.getmtime(s) > os.path.getmtime(out) for s in src):
-        subprocess.run(["g++", "-x", "c++", "-std=c++17", "-DT4_EMU", "-O2", "-g", "-ffp-contract=off", "-fPIC", "-shared",
-                        "-o", out, src[0]], check=True)
-    lib = api.Lib(out, "t4emu_")
+    lib = api.Lib(__graft_entry__.build_emu(), "t4emu_")
     lib.check(lib.init(0, 2 << 30))
     return lib
 
@@ -55,9 +48,20 @@ def gpu_lib():
     return lib
 
 
-@pytest.fixture(scope="session")
-def ref():
+@pytest.fixture
+def ref(request):
+    """The reference's classes: live from oracle/_ref/libt4ref.so where it is built, else the results recorded from it
+    under tests/golden/ref (tests/refharness.py)."""
+    import refharness
+    refharness.use_tape(request.node.nodeid)
+    yield refharness
+    refharness.end_tape()
+
+
+@pytest.fixture
+def ref_live():
+    """The compiled reference itself, for tests of the oracle (they have nothing to check without it)."""
     import refharness
     if not refharness.available():
-        pytest.skip("oracle/_ref/libt4ref.so not built (make -C oracle)")
+        pytest.skip("oracle/_ref/libt4ref.so not built: needs the reference sources (make -C oracle)")
     return refharness

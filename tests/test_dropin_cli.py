@@ -2,10 +2,14 @@
 repository's C-ABI library must write the same _raw.out, _final.out and _assembled_reads.fa as the stock `trust4`
 (oracle/_ref/trust4) -- flags, file formats and `run-trust4 --stage 1` compatibility included (SURVEY.md 8b).
 
-CPU variant: the binding linked against the test emulation of the engine (needs the reference sources to build).
-GPU variant: integration/_build/trust4_gpu, prebuilt by __graft_entry__.build() where the reference sources exist;
-both binaries run on the box itself on freshly generated synthetic FASTQ, so nothing under /root/reference is read."""
+CPU variant: integration/_build/trust4_emu{,_batch}, the binding linked against the test emulation of the engine.
+GPU variant: integration/_build/trust4_gpu{,_batch}, linked against libtrust4_b200.so.
+All of them, and the stock binary, are compiled from the reference's main.cpp, which is not part of this repository:
+__graft_entry__.build() builds them where the reference sources exist, and the tests use them wherever they were built.
+Inputs are synthetic FASTQ generated here, or the reference's shipped example (tests/golden/*.gz)."""
+import gzip
 import os
+import shutil
 import subprocess
 
 import pytest
@@ -14,7 +18,7 @@ from trust4_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STOCK = os.path.join(ROOT, "oracle", "_ref", "trust4")
-REF = "/root/reference"
+GOLD = os.path.join(ROOT, "tests", "golden")
 SUFFIXES = ("_raw.out", "_final.out", "_assembled_reads.fa")
 
 
@@ -57,6 +61,16 @@ def write_barcode_inputs(tmp, nreads=1500, nclones=24, n_barcodes=6, seed=23):
     return ["-f", fa, "-u", os.path.join(tmp, "reads.fq"), "--barcode", os.path.join(tmp, "bc.fa")]
 
 
+def example_inputs(tmp):
+    """BASELINE.json configs[0]: the reference's shipped example, example_1.fq + example_2.fq -f hg38_bcrtcr.fa."""
+    paths = []
+    for name in ("hg38_bcrtcr.fa", "example_1.fq", "example_2.fq"):
+        paths.append(os.path.join(tmp, name))
+        with gzip.open(os.path.join(GOLD, name + ".gz")) as src, open(paths[-1], "wb") as dst:
+            shutil.copyfileobj(src, dst)
+    return ["-f", paths[0], "-1", paths[1], "-2", paths[2]]
+
+
 def run_and_compare(binary, args, tmp, extra=(), env=None):
     for exe, tag in ((STOCK, "stock"), (binary, "dropin")):
         e = dict(os.environ, **env) if (env and exe is binary) else None
@@ -68,32 +82,29 @@ def run_and_compare(binary, args, tmp, extra=(), env=None):
         assert len(a) > 0 and a == b, suf
 
 
+def prebuilt(name):
+    """integration/_build/<name> and the stock binary, as __graft_entry__.build() left them (both need the reference sources)."""
+    binary = os.path.join(ROOT, "integration", "_build", name)
+    if not (os.path.exists(binary) and os.path.exists(STOCK)):
+        pytest.skip("drop-in / stock binaries not built: they are compiled from the reference's main.cpp")
+    return binary
+
+
 @pytest.fixture(scope="module")
 def emu_binary(emu_lib):
-    if not os.path.exists(os.path.join(REF, "main.cpp")):
-        pytest.skip("reference sources not present (needed to compile main.cpp)")
-    if not os.path.exists(STOCK):
-        pytest.skip("oracle/_ref/trust4 not built")
-    subprocess.run(["make", "-C", os.path.join(ROOT, "integration"), "_build/trust4_emu"], check=True, stdout=subprocess.DEVNULL)
-    return os.path.join(ROOT, "integration", "_build", "trust4_emu")
+    return prebuilt("trust4_emu")
 
 
 @pytest.fixture(scope="module")
 def emu_batch_binary(emu_lib):
     """The batch route: main.cpp + one inserted line per offloaded pass (integration/make_batch_main.py), T4_STREAMS selects the device streams."""
-    if not os.path.exists(os.path.join(REF, "main.cpp")):
-        pytest.skip("reference sources not present (needed to compile main.cpp)")
-    if not os.path.exists(STOCK):
-        pytest.skip("oracle/_ref/trust4 not built")
-    subprocess.run(["make", "-C", os.path.join(ROOT, "integration"), "_build/trust4_emu_batch"], check=True, stdout=subprocess.DEVNULL)
-    return os.path.join(ROOT, "integration", "_build", "trust4_emu_batch")
+    return prebuilt("trust4_emu_batch")
 
 
 def test_batch_emu_shipped_example(emu_batch_binary, tmp_path):
     """BASELINE.json configs[0] through the batch route, one stream: the device runs the whole loop + rescue pass in one
     launch, the driver's own loop replays its decisions; all three output files byte-identical to the stock binary."""
-    args = ["-f", REF + "/hg38_bcrtcr.fa", "-1", REF + "/example/example_1.fq", "-2", REF + "/example/example_2.fq"]
-    run_and_compare(emu_batch_binary, args, str(tmp_path), env={"T4_STREAMS": "1"})
+    run_and_compare(emu_batch_binary, example_inputs(str(tmp_path)), str(tmp_path), env={"T4_STREAMS": "1"})
 
 
 def test_batch_emu_synthetic(emu_batch_binary, tmp_path):
@@ -131,7 +142,7 @@ def test_batch_emu_annotate_on_device(emu_batch_binary, tmp_path, case):
     if case == "synthetic":
         args = write_inputs(tmp, 1500, 50, 33)
     elif case == "example":
-        args = ["-f", REF + "/hg38_bcrtcr.fa", "-1", REF + "/example/example_1.fq", "-2", REF + "/example/example_2.fq"]
+        args = example_inputs(tmp)
     else:
         args = write_inputs(tmp, 800, 25, 34)
         extra = ["--trimLevel", "2", "--skipMateExtension"]
@@ -218,8 +229,7 @@ def test_batch_emu_sharded_runs(emu_batch_binary, tmp_path):
 
 def test_dropin_emu_shipped_example(emu_binary, tmp_path):
     """BASELINE.json configs[0]: example_1.fq + example_2.fq -f hg38_bcrtcr.fa, -t 1."""
-    args = ["-f", REF + "/hg38_bcrtcr.fa", "-1", REF + "/example/example_1.fq", "-2", REF + "/example/example_2.fq"]
-    run_and_compare(emu_binary, args, str(tmp_path))
+    run_and_compare(emu_binary, example_inputs(str(tmp_path)), str(tmp_path))
 
 
 def test_dropin_emu_synthetic(emu_binary, tmp_path):
@@ -245,17 +255,13 @@ def test_dropin_emu_barcodes(emu_binary, tmp_path, extra):
 
 @pytest.mark.gpu
 def test_dropin_gpu_barcodes(tmp_path):
-    binary = os.path.join(ROOT, "integration", "_build", "trust4_gpu")
-    if not (os.path.exists(binary) and os.path.exists(STOCK)):
-        pytest.skip("prebuilt drop-in / stock binaries not present")
+    binary = prebuilt("trust4_gpu")
     run_and_compare(binary, write_barcode_inputs(str(tmp_path)), str(tmp_path), extra=("--contigMinCov", "4"))
 
 
 @pytest.mark.gpu
 def test_batch_gpu_synthetic_and_barcodes(tmp_path):
-    binary = os.path.join(ROOT, "integration", "_build", "trust4_gpu_batch")
-    if not (os.path.exists(binary) and os.path.exists(STOCK)):
-        pytest.skip("prebuilt drop-in / stock binaries not present")
+    binary = prebuilt("trust4_gpu_batch")
     a = tmp_path / "a"
     b = tmp_path / "b"
     a.mkdir()
@@ -266,7 +272,5 @@ def test_batch_gpu_synthetic_and_barcodes(tmp_path):
 
 @pytest.mark.gpu
 def test_dropin_gpu_synthetic(tmp_path):
-    binary = os.path.join(ROOT, "integration", "_build", "trust4_gpu")
-    if not (os.path.exists(binary) and os.path.exists(STOCK)):
-        pytest.skip("prebuilt drop-in / stock binaries not present")
+    binary = prebuilt("trust4_gpu")
     run_and_compare(binary, write_inputs(str(tmp_path)), str(tmp_path))

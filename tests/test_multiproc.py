@@ -10,13 +10,14 @@ import torch.multiprocessing as mp
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _worker(rank, world, port, emu_path, q):
+def _worker(rank, world, port, emu_path, q, test_id):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import numpy as np
     import torch.distributed as dist
     from trust4_b200 import api, synth, dist as tdist
     import refharness as rh
+    rh.use_tape("%s-rank%d" % (test_id, rank))
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -45,15 +46,16 @@ def _worker(rank, world, port, emu_path, q):
     t = torch.from_numpy(cnt)
     dist.all_reduce(t)
     assert int(t.item()) == tot
+    rh.end_tape()
     q.put((rank, tot))
     dist.destroy_process_group()
 
 
-def test_two_rank_shard_and_allgather(emu_lib, ref):
+def test_two_rank_shard_and_allgather(emu_lib, ref, request):
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29500 + os.getpid() % 1000
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, emu_lib.path, q)) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, emu_lib.path, q, request.node.nodeid)) for r in range(2)]
     for p in procs:
         p.start()
     for p in procs:
